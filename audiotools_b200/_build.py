@@ -9,6 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(CSRC, "libb2a.so")
+STAMP = os.path.join(CSRC, ".libb2a.stamp")
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC",
@@ -33,9 +34,12 @@ def _digest(files):
 def build(force: bool = False, verbose: bool = False) -> str:
     """Build (if stale) and return the path of libb2a.so.  Safe to call from several processes at once (the ranks of a
     torchrun launch, the two ranks of a gloo test): an exclusive file lock serialises the builders and the library is
-    moved into place atomically, so a concurrent importer never sees a half-written file."""
+    moved into place atomically, so a concurrent importer never sees a half-written file.  An up-to-date library is
+    returned without writing anything, so a built tree may be read-only."""
     import fcntl
 
+    if not force and _up_to_date(_digest(_deps())):
+        return OUT
     with open(os.path.join(CSRC, ".build.lock"), "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
         try:
@@ -44,13 +48,21 @@ def build(force: bool = False, verbose: bool = False) -> str:
             fcntl.flock(lock, fcntl.LOCK_UN)
 
 
+def _deps():
+    return sorted(glob.glob(os.path.join(CSRC, "*.cu"))) + sorted(glob.glob(os.path.join(CSRC, "*.h"))) + sorted(
+        glob.glob(os.path.join(CSRC, "*.cuh"))) + [os.path.join(os.path.dirname(HERE), "include", "b2a.h")]
+
+
+def _up_to_date(dig: str) -> bool:
+    """The library exists and the stamp written after it names the digest ``dig`` of the current sources."""
+    return os.path.exists(OUT) and os.path.exists(STAMP) and open(STAMP).read() == dig
+
+
 def _build_locked(force: bool, verbose: bool) -> str:
-    srcs = sorted(glob.glob(os.path.join(CSRC, "*.cu")))
-    deps = srcs + sorted(glob.glob(os.path.join(CSRC, "*.h"))) + sorted(glob.glob(os.path.join(CSRC, "*.cuh"))) + [
-        os.path.join(os.path.dirname(HERE), "include", "b2a.h")]
-    stamp = os.path.join(CSRC, ".libb2a.stamp")
+    deps = _deps()
+    srcs = [d for d in deps if d.endswith(".cu")]
     dig = _digest(deps)
-    if not force and os.path.exists(OUT) and os.path.exists(stamp) and open(stamp).read() == dig:
+    if not force and _up_to_date(dig):
         return OUT
     nvcc = _nvcc()
     objs, procs = [], []
@@ -69,7 +81,7 @@ def _build_locked(force: bool, verbose: bool) -> str:
     cmd = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", tmp] + objs
     subprocess.check_call(cmd)
     os.replace(tmp, OUT)
-    with open(stamp, "w") as f:
+    with open(STAMP, "w") as f:
         f.write(dig)
     return OUT
 

@@ -2,8 +2,11 @@
 """bench.py -- the BASELINE.json metric: clips/sec for 10 s @ 44.1 kHz stereo clips through
 LUFS-normalise (-24) + log-mel (n_fft 2048, hop 512, 128 mels)  [BASELINE.json configs[1]].
 
-  python bench.py [--gpus N --steps K --warmup W]                    our arm (CUDA, one rank per GPU)
+  python bench.py [--gpus N --steps K --warmup W] [--dump-outputs DIR] our arm (CUDA, one rank per GPU)
   python bench.py --impl reference [--gpus N --steps K --warmup W]    the reference's CPU path (oracle port)
+
+--dump-outputs DIR writes what the last timed step returned on rank 0 (see dump_sample) as DIR/<name>.npy, float32:
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 One "step" = one pass of the hot path over one batch of 64 clips per GPU (weak scaling): the
 loudness kernels, then the fused gain + STFT + mel + log kernel.  Outputs per step: normalised
@@ -49,6 +52,27 @@ def make_batch(B, seed, device="cpu"):
     x = (0.1 * torch.randn(B, C, T, generator=g)).clamp(-1, 1)
     x = x * (0.05 + 0.95 * torch.rand(B, 1, 1, generator=g))
     return x.float().to(device)
+
+
+DUMP_MAX_ELEMS = 1 << 22  # 16 MiB of float32 per array: a step's two large outputs and three [B] vectors stay < 64 MB
+
+
+def dump_sample(arrays):
+    """Host float32 copies of the device tensors ``arrays``.  One with more than DUMP_MAX_ELEMS elements is replaced by
+    DUMP_MAX_ELEMS of its flattened elements, one drawn from each of that many equal strides by a generator seeded
+    with 0: the same shape always gives the same positions."""
+    import numpy as np
+    import torch
+
+    out = {}
+    for name, t in arrays.items():
+        n = t.numel()
+        if n > DUMP_MAX_ELEMS:
+            stride = n // DUMP_MAX_ELEMS
+            idx = np.arange(DUMP_MAX_ELEMS) * stride + np.random.default_rng(0).integers(0, stride, DUMP_MAX_ELEMS)
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        out[name] = t.float().cpu().numpy()
+    return out
 
 
 # ----------------------------------------------------------------------------------------------
@@ -304,9 +328,15 @@ def run_ours(args):
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0.record()
         for i in range(args.steps):
-            step(args.warmup + i, timed=True)
+            last = step(args.warmup + i, timed=True)
+            if i + 1 < args.steps:
+                last = None  # freed before the next step, whose outputs then reuse the memory
         t1.record()
         torch.cuda.synchronize()
+        dumped = None
+        if args.dump_outputs and rank == 0:  # the last timed step's results: dict(lufs, loud, gain, mel, scaled)
+            dumped = dump_sample({k: v for d in (last[1], last[0]) for k, v in d.items() if v is not None})
+        last = None
         w_timed1 = time.perf_counter()
         ms_rank = t0.elapsed_time(t1)
         launches = eng.launches - launches0 + (exchange.launches - xl0 if exchange is not None else 0)
@@ -492,6 +522,12 @@ def run_ours(args):
         "sustained": sus_line, "exchange": exchange_line,
         "gpu_launches": launches, "clocks": clk,
     }
+    if dumped is not None:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -511,7 +547,15 @@ def main():
     ap.add_argument("--tc", action="store_true", help="use the opt-in tensor-core spectral kernel (A/B measurements)")
     ap.add_argument("--e2e-features-only", action="store_true",
                     help="e2e leg copies back log-mel + LUFS only (not the normalised waveform)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs (rank 0) to DIR/<name>.npy: lufs, loud, gain [B], "
+                         "mel (log-mel) and scaled (normalised waveform); an array of more than 2**22 elements as a "
+                         "fixed, seeded sample of that many")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps our arm's outputs (--impl ours)")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
